@@ -119,13 +119,11 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
-def cpu_reference_step_time(threads, reps=1, budget_s=None, min_reps=1):
+def cpu_reference_step_time(threads, reps=1):
     """The reference's own CPU path: the UNMODIFIED `models_painter.painter_vit_large_patch16_input896x448_win_dec64_
-    8glb_sl1()` module (staged copy under baseline/_ref, scripts/stage_reference.py; loaded through oracle/ref_loader)
+    8glb_sl1()` module (staged copy under oracle/_ref, oracle/stage_reference.py; loaded through oracle/ref_loader)
     in torch-CPU eager fp32, train mode, B=1 896x448 forward + backward on `threads` host threads.  Falls back to the
-    oracle port (kind "port") only if the staged tree is missing.  With `budget_s` the loop stops early once that much
-    wall time is spent (after at least `min_reps` steps), so the CPU legs stay bounded whatever --steps is.
-    Returns (times, kind)."""
+    oracle port (kind "port") only if the staged tree is missing.  Returns (times of the `reps` steps, kind)."""
     import torch
     from oracle import painter_oracle as po
     from oracle import ref_loader
@@ -160,8 +158,6 @@ def cpu_reference_step_time(threads, reps=1, budget_s=None, min_reps=1):
         t0 = time.perf_counter()
         one()
         times.append(time.perf_counter() - t0)
-        if budget_s is not None and len(times) >= min_reps and sum(times) > budget_s:
-            break
     return times, kind
 
 
@@ -174,7 +170,7 @@ def reference_cuda_eager(dev, host, steps):
     from oracle import ref_loader
     from oracle.synth import synth_state_dict
     if not ref_loader.available():
-        return {"unavailable": "reference tree not staged (scripts/stage_reference.py)"}
+        return {"unavailable": "reference tree not staged (oracle/stage_reference.py)"}
     torch.cuda.empty_cache()
     model = ref_loader.models_painter().painter_vit_large_patch16_input896x448_win_dec64_8glb_sl1()
     model.load_state_dict(synth_state_dict(po.PainterConfig(), 0), strict=True)
@@ -213,8 +209,8 @@ def run_reference(args):
     if rank != 0:
         return
     threads = min(os.cpu_count() or 1, 32)   # beyond ~32 threads torch-CPU eager slows down (oversubscription)
-    # bounded sample: one warm-up step, then up to --steps timed steps or ~150 s of CPU work, whichever comes first
-    t, kind = cpu_reference_step_time(threads, reps=1 + args.steps, budget_s=150.0, min_reps=2)
+    # one warm-up step, then --steps timed steps
+    t, kind = cpu_reference_step_time(threads, reps=1 + args.steps)
     t = t[1:]
     ms = 1e3 * sum(t) / len(t)
     val = 1.0 / (ms / 1e3)
@@ -264,7 +260,7 @@ def run_seggpt_reference(args):
     model.seg_type = "instance"
     img, tgt = _seggpt_inputs()
     times = []
-    for _ in range(1 + min(args.steps, 5)):
+    for _ in range(1 + args.steps):
         t0 = time.perf_counter()
         se.run_one_image(img, tgt, model, torch.device("cpu"))
         times.append(time.perf_counter() - t0)
@@ -312,7 +308,7 @@ def run_seggpt(args):
                 p.normal_(std=0.02)
     model.seg_type = "instance"
     img, tgt = _seggpt_inputs()
-    steps, W_steps = max(args.steps, 1), max(args.warmup, 3)
+    steps, W_steps = args.steps, max(args.warmup, 3)
     x = torch.from_numpy(img).permute(0, 3, 1, 2).float().contiguous().to(dev)
     t = torch.from_numpy(tgt).permute(0, 3, 1, 2).float().contiguous().to(dev)
 
@@ -364,7 +360,7 @@ def run_seggpt(args):
     # fp32-accurate mode first (reported as an extra block), then the headline bf16 mode under the clock sampler
     acc = None
     if args.precision in ("both", "fp32"):
-        a_eager, a_graph, a_e2e, a_launches, _ = measure("fp32", max(steps, 3))
+        a_eager, a_graph, a_e2e, a_launches, _ = measure("fp32", steps)
         acc = {"ms_per_step": a_graph, "value": world * 1e3 / a_graph, "eager_ms_per_step": a_eager,
                "e2e_ms_per_step": a_e2e, "e2e_value": world * 1e3 / a_e2e, "kernels_per_forward": int(a_launches),
                "note": "model.precision = 'fp32': split-bf16 (3 terms, 6 products) tensor-core GEMMs, fp32 softmax / "
@@ -373,15 +369,19 @@ def run_seggpt(args):
     clocks = ClockSampler(local)
     if rank == 0:
         clocks.start()
-    ms_eager, ms_graph, ms_e2e, launches, out = measure("bf16", steps * 5)
+    ms_eager, ms_graph, ms_e2e, launches, out = measure("bf16", steps)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)      # what run_one_image returned in the last timed e2e step
+        np.save(os.path.join(args.dump_outputs, "result.npy"), out.numpy().astype(np.float64))
     ms_graph, ms_e2e, ms_eager = dist_utils.max_over_ranks([ms_graph, ms_e2e, ms_eager], device=dev)
     if rank == 0:
         peak, peak_src = _peaks()
         achieved = FLOPS_SEGGPT_FWD / (ms_graph / 1e3) / 1e12
         line = {
             "metric": "images/sec SegGPT ViT-L in-context inference (1 prompt + 1 target 448x448)",
-            "value": world * 1e3 / ms_graph, "unit": "images/s", "n_gpus": world, "steps": steps * 5, "warmup": W_steps,
+            "value": world * 1e3 / ms_graph, "unit": "images/s", "n_gpus": world, "steps": steps, "warmup": W_steps,
             "ms_per_step": ms_graph, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "bf16",
             "data": "synthetic",
             "config": {"workload": "SegGPT ViT-L in-context segmentation inference, 1 prompt pair + 1 target 448x448 "
@@ -394,7 +394,7 @@ def run_seggpt(args):
                     "h2d_bytes_per_step": int(img.nbytes + tgt.nbytes), "d2h_bytes_per_step": int(out.numel() * 8),
                     "call": "painter_b200.seggpt_engine.run_one_image(img, tgt, model, device): numpy float64 canvases in, "
                             "de-normalised [448,448,3] float64 result on the host out (wall clock incl. both copies)"},
-            "gpu_launches": int(launches) * steps * 5,
+            "gpu_launches": int(launches) * steps,
             "roofline": {"bound": "tensor", "kernel": "whole forward (tcgen05 GEMMs + fused attention), one graph replay",
                          "achieved": achieved, "peak": peak, "unit": "TFLOP/s", "frac": achieved / peak,
                          "peak_source": peak_src, "algorithmic_per_launch": FLOPS_SEGGPT_FWD, "traffic": None},
@@ -414,6 +414,29 @@ def run_seggpt(args):
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_PARAM_SAMPLES = 1024            # per parameter tensor, at positions seeded by the tensor's index
+DUMP_PRED_MAX = 8 * 1568 * 768        # logits values written whole (the headline batch); a seeded sample beyond that
+
+
+def dump_outputs(out_dir, loss, pred, mask, model):
+    """What one training step hands back to its caller, as float32 .npy files (about 40 MB at the headline batch):
+    loss.npy, pred.npy (the logits, [B, tokens, 768]), mask.npy and params_sample.npy, the parameters after the
+    optimizer update at DUMP_PARAM_SAMPLES seeded positions per tensor (named_parameters() order)."""
+    import numpy as np
+    import torch
+    from oracle.synth import sample_positions
+    os.makedirs(out_dir, exist_ok=True)
+    p = pred.detach().float()
+    if p.numel() > DUMP_PRED_MAX:
+        p = p.reshape(-1)[sample_positions(p.numel(), DUMP_PRED_MAX, 0).to(p.device)]
+    params = [t.detach().reshape(-1)[sample_positions(t.numel(), DUMP_PARAM_SAMPLES, i).to(t.device)].float()
+              for i, t in enumerate(model.parameters())]
+    arrays = {"loss": loss.detach().float().reshape(1), "pred": p, "mask": mask.detach().float(),
+              "params_sample": torch.cat(params)}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
 
 
 def main():
@@ -447,7 +470,15 @@ def main():
                     help="1: the e2e step is painter_b200.train_utils.GraphedTrainStep (forward + backward + AdamW as one "
                          "CUDA-graph replay; N = 1 with the pk optimizer); 0: the reference loop's eager launches")
     ap.add_argument("--no-optimizer", action="store_true", help="diagnostic only; the reported step includes AdamW")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last one computed as DIR/<name>.npy: train / long: "
+                         "loss, logits, mask, a seeded sample of the updated parameters; seggpt: run_one_image's "
+                         "result")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what painter_b200 computed; it has no meaning with --impl reference")
     if args.workload == "seggpt":
         return run_seggpt(args)
     if args.impl == "reference":
@@ -537,12 +568,12 @@ def main():
     def step(batch, read_loss):
         imgs, tgts, mask, valid = batch
         with torch.autocast("cuda", dtype=torch.bfloat16):
-            loss, _, _ = net(imgs, tgts, bool_masked_pos=mask, valid=valid)
+            loss, pred, bmask = net(imgs, tgts, bool_masked_pos=mask, valid=valid)
         loss.backward()
         if not args.no_optimizer:
             opt.step()
         opt.zero_grad(set_to_none=True)
-        return loss.item() if read_loss else None
+        return loss.item() if read_loss else (loss, pred, bmask)
 
     def sync():
         if world > 1:
@@ -576,12 +607,15 @@ def main():
     e0.record()
     for i in range(args.steps):
         record["on"] = i in sampled
-        step(resident, False)
+        last = step(resident, False)
     e1.record()
     sync()
     launches = _lib.launch_count() - n0
     record["on"] = False
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last, model)
+    del last
     # ---------------- timed region 2: end to end through the public API, the reference loop's way ----------------
     # strict = engine_train.train_one_epoch verbatim (engine_train.py:52-93): every step copies its batch from pinned
     # host memory with .to(device, non_blocking=True) on the compute stream, calls the module under autocast, reads

@@ -5,8 +5,8 @@ __graft_entry__.smoke() and by bench.py's cpu_baseline / --impl reference legs; 
 (painter_b200/*) never imports it and has no CPU fallback.
 
 Parity status: PINNED — tests/test_oracle_golden.py checks this restatement against golden vectors
-produced by executing the unmodified reference (oracle/make_golden.py, run in the authoring container
-where /root/reference exists) and, when the reference is present, against the live reference module.
+produced by executing the unmodified reference (oracle/make_golden.py), at toy geometries and at the
+benchmark geometry.
 The reference itself ships no tests or golden vectors (SURVEY.md §4).
 
 It restates, as a pure function of a reference-format state_dict:

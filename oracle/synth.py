@@ -99,6 +99,21 @@ def synth_inputs(cfg: PainterConfig, B, seed, mask_kind="random", valid_kind="on
     return imgs, tgts, mask, valid
 
 
+def compact(t, n=4096, seed=0):
+    """A reference tensor too large to store whole: its size, exact sum of squares and max |x|, and its values at n
+    positions drawn (with replacement) from a generator seeded by `seed`; sample_positions() regenerates them."""
+    t = t.detach().float().cpu().reshape(-1)
+    idx = sample_positions(t.numel(), n, seed)
+    return {"numel": t.numel(), "n": n, "seed": seed, "val": t[idx].clone(),
+            "sumsq": float(t.double().pow(2).sum()), "absmax": float(t.abs().max())}
+
+
+def sample_positions(numel, n, seed):
+    if numel <= n:
+        return torch.arange(numel)
+    return torch.randint(numel, (n,), generator=torch.Generator().manual_seed(seed))
+
+
 def fingerprint(sd):
     """Cheap checksum guarding against RNG drift between torch builds."""
     s = 0.0

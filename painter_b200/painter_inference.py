@@ -26,8 +26,9 @@ def run_one_image(img, tgt, size, model, out_path, device):
     from PIL import Image
     device = torch.device(device)
     net = model.module if hasattr(model, "module") else model
-    x = torch.as_tensor(img).unsqueeze(0).to(device, non_blocking=True)
-    t = torch.as_tensor(tgt).unsqueeze(0).to(device, non_blocking=True)
+    # pk_nhwc_to_nchw_f32 reads packed NHWC: .to() keeps a strided (e.g. permuted) array's strides, so pack it
+    x = torch.as_tensor(img).unsqueeze(0).to(device, non_blocking=True).contiguous()
+    t = torch.as_tensor(tgt).unsqueeze(0).to(device, non_blocking=True).contiguous()
     _, H, W, _ = x.shape
     xin = torch.empty((1, 3, H, W), dtype=torch.float32, device=device)
     tin = torch.empty((1, 3, H, W), dtype=torch.float32, device=device)

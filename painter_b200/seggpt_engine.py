@@ -122,7 +122,8 @@ def run_one_image(img, tgt, model, device):
     x = torch.as_tensor(img)
     t = torch.as_tensor(tgt)
     P, H, W, _ = x.shape
-    xd, td = x.to(device, non_blocking=True), t.to(device, non_blocking=True)
+    # pk_nhwc_to_nchw_f32 reads packed NHWC: .to() keeps a strided (e.g. permuted) array's strides, so pack it
+    xd, td = x.to(device, non_blocking=True).contiguous(), t.to(device, non_blocking=True).contiguous()
     xin = torch.empty((P, 3, H, W), dtype=torch.float32, device=device)
     tin = torch.empty((P, 3, H, W), dtype=torch.float32, device=device)
     for src, dst in ((xd, xin), (td, tin)):

@@ -1,5 +1,5 @@
-"""TEST INFRASTRUCTURE: the UNMODIFIED reference modules (oracle/ref_loader.py: /root/reference here, the staged
-byte-for-byte copy baseline/_ref on the GPU box) loaded with the same synthetic weights as the painter_b200 module.
+"""TEST INFRASTRUCTURE: the UNMODIFIED reference modules (oracle/ref_loader.py: $PAINTER_REFERENCE or the
+staged byte-for-byte copy oracle/_ref) loaded with the same synthetic weights as the painter_b200 module.
 """
 from contextlib import contextmanager
 from functools import partial

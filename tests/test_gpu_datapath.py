@@ -1,17 +1,16 @@
 """GPU data-path kernels (SURVEY §8 f.4) against the unmodified reference: the block-mask generator keeps the
 reference's invariants and statistics (its random source differs, so parity is distributional), the `valid` maps are
-bit-identical to PairDataset.__getitem__ (driven on temporary image files)."""
-import json
-import os
-import random
-
+bit-identical to PairDataset.__getitem__ (driven on temporary image files).  The reference side is stored in
+tests/golden/ref_datapath.pt (`python -m oracle.make_golden datapath`)."""
 import numpy as np
 import pytest
 import torch
 
-from oracle import ref_loader
+from oracle.make_golden import to_normalised
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_loader.available(), reason="reference tree not staged")]
+from _common import load_golden
+
+pytestmark = pytest.mark.gpu
 
 
 def _blockiness(m):
@@ -21,24 +20,20 @@ def _blockiness(m):
 
 def test_block_masks_invariants_and_statistics_vs_reference_generator():
     from painter_b200.data_gpu import DeviceMaskingGenerator
-    MG = ref_loader.masking_generator().MaskingGenerator
+    ref = load_golden("ref_datapath.pt")["masks"]
     h, w, target = 56, 28, 784
-    ref = MG((h, w), num_masking_patches=target, max_num_patches=392, min_num_patches=16)     # main_train.py:256-260
     ours = DeviceMaskingGenerator((h, w), num_masking_patches=target, max_num_patches=392, min_num_patches=16)
     n = 1024
     mo = torch.cat([ours(256, seed=100 + k) for k in range(n // 256)]).cpu().numpy()
     assert mo.shape == (n, h, w) and set(np.unique(mo)) <= {0, 1}
     assert (mo.reshape(n, -1).sum(1) == target).all()                                  # exact count, every sample
     assert len({m.tobytes() for m in mo}) == n                                         # all different
-    random.seed(0)
-    np.random.seed(0)
-    mr = np.stack([ref() for _ in range(n)])
-    assert (mr.reshape(n, -1).sum(1) == target).all()
-    # same structure: block-iness (neighbour agreement) and the spatial masking profile
-    assert abs(_blockiness(mo) - _blockiness(mr)) < 0.01, (_blockiness(mo), _blockiness(mr))
-    assert np.abs(mo.mean(0) - mr.mean(0)).max() < 0.08
-    assert np.abs(mo.mean((0, 2)) - mr.mean((0, 2))).max() < 0.03                      # per-row marginal
-    assert np.abs(mo.mean((0, 1)) - mr.mean((0, 1))).max() < 0.03                      # per-column marginal
+    # same structure as 1024 draws of the reference generator: block-iness (neighbour agreement) and the spatial
+    # masking profile
+    assert abs(_blockiness(mo) - ref["blockiness"]) < 0.01, (_blockiness(mo), ref["blockiness"])
+    assert np.abs(mo.mean(0) - ref["mean_map"].numpy()).max() < 0.08
+    assert np.abs(mo.mean((0, 2)) - ref["row_marginal"].numpy()).max() < 0.03          # per-row marginal
+    assert np.abs(mo.mean((0, 1)) - ref["col_marginal"].numpy()).max() < 0.03          # per-column marginal
     # the half-mask alternative (pairdataset.py:183-186)
     half = DeviceMaskingGenerator((h, w), target, max_num_patches=392, min_num_patches=16, half_mask_ratio=1.0)(4, 7)
     want = torch.zeros(h, w, dtype=torch.int32)
@@ -49,53 +44,18 @@ def test_block_masks_invariants_and_statistics_vs_reference_generator():
     assert 0.06 < frac < 0.14, frac
 
 
-def test_valid_maps_bit_identical_to_pairdataset(tmp_path):
-    from PIL import Image
+def test_valid_maps_bit_identical_to_pairdataset():
+    """PairDataset.__getitem__ on the 12 image pairs of oracle.make_golden.datapath_pairs (all six task types, black
+    regions, an almost empty pose target, an empty instance target): its targets, rebuilt from the stored pixels, give
+    painter_b200's valid maps bit for bit equal to the ones it returned."""
     from painter_b200.data_gpu import combine_pairs, valid_maps
-    PD = ref_loader.pairdataset()
-    MG = ref_loader.masking_generator().MaskingGenerator
-    rng = np.random.RandomState(0)
-    types = ["nyuv2_image2depth", "ade20k_image2semantic", "coco_image2panoptic_sem_seg", "coco_image2pose",
-             "coco_image2panoptic_inst", "ssid_image2denoise"]
-    H = W = 64
-    pairs = []
-    for t in types:
-        for k in range(2):
-            img = rng.randint(0, 256, (H, W, 3)).astype(np.uint8)
-            tgt = rng.randint(0, 256, (H, W, 3)).astype(np.uint8)
-            tgt[: H // 2, : W // 3] = 0                       # black region -> below every threshold
-            if "pose" in t and k == 0:
-                tgt[:] = 0                                    # nearly no foreground -> valid = 0 branch
-                tgt[0, 0] = 200
-            if "inst" in t and k == 1:
-                tgt[:] = 0
-            ip, tp = f"{t}_{k}_img.png", f"{t}_{k}_tgt.png"
-            Image.fromarray(img).save(tmp_path / ip)
-            Image.fromarray(tgt).save(tmp_path / tp)
-            pairs.append({"image_path": ip, "target_path": tp, "type": t})
-    jp = tmp_path / "pairs.json"
-    json.dump(pairs, open(jp, "w"))
-    mean = torch.tensor([0.485, 0.456, 0.406])[:, None, None]
-    std = torch.tensor([0.229, 0.224, 0.225])[:, None, None]
-
-    def tf(img, tgt, i1, i2):
-        f = lambda im: (torch.from_numpy(np.array(im)).permute(2, 0, 1).float() / 255.0 - mean) / std
-        return f(img), f(tgt)
-
-    ds = PD.PairDataset(str(tmp_path), [str(jp)], transform=tf, masked_position_generator=MG((8, 4), 16, 4),
-                        use_two_pairs=True, half_mask_ratio=0.0)
-    random.seed(1)
-    torch.manual_seed(1)
-    tg, vd, tp = [], [], []
-    for i in range(len(ds)):
-        image, target, mask, valid = ds[i]
-        assert tuple(target.shape) == (3, 2 * H, W)
-        tg.append(target)
-        vd.append(valid)
-        tp.append(pairs[i]["type"])
-    ours = valid_maps(torch.stack(tg).cuda().contiguous(), tp)
+    ref = load_golden("ref_datapath.pt")
+    tg = torch.stack([to_normalised(u) for u in ref["targets_u8"]])
+    assert tuple(tg.shape[1:]) == (3, 128, 64)
+    ours = valid_maps(tg.cuda().contiguous(), ref["types"])
+    vd = ref["valid"].float()
     for i, v in enumerate(vd):
-        assert torch.equal(ours[i].cpu(), v), (tp[i], (ours[i].cpu() != v).sum())
-    assert {float(x) for x in torch.stack(vd).unique()} == {0.0, 1.0, 10.0}       # all three branches were exercised
-    a, b = torch.randn(2, 3, 8, 4), torch.randn(2, 3, 8, 4)
-    assert torch.equal(combine_pairs(a, b)[0], ds._combine_images(a[0], b[0]))
+        assert torch.equal(ours[i].cpu(), v), (ref["types"][i], (ours[i].cpu() != v).sum())
+    assert {float(x) for x in vd.unique()} == {0.0, 1.0, 10.0}       # all three branches were exercised
+    c = ref["combine"]
+    assert torch.equal(combine_pairs(c["a"], c["b"])[0], c["out"])
