@@ -57,7 +57,7 @@ typedef struct {
   int ld_aux;         /* row stride of aux (elements) */
   int rows_per_group; /* rows sharing one rowscale entry */
   int accumulate;     /* PK_EPI_F32: 0 overwrite, 1 out += , 2 out zero-initialised, split-K atomics */
-  float alpha;
+  float alpha;        /* scales acc (alpha == 0 is taken as 1, so a zero-initialised struct computes acc) */
   int ps_h, ps_w, ps_p, ps_c; /* pixel shuffle geometry: token grid h x w, patch p, channels c */
 } PkEpilogue;
 
@@ -141,6 +141,8 @@ int pk_ensemble_resid(const float* a, const float* z, float* out, int G, int P, 
  * Fused attention with decomposed relative-position bias (models_painter.py:73-86 + util/vitdet_utils.py:
  * 63-125).  qkv bf16 [B*h*w, 3*heads*64] with columns (3, head, 64); th/tw = pk_relpos_table_bf16 outputs
  * (bf16, zero-padded to th_pad/tw_pad rows, multiples of 16); w must divide 112 (2,4,7,8,14,28,56).
+ * Limits: fwd th_pad <= 256 (h <= 128), bwd th_pad <= 224 (h <= 112), both tw_pad <= 112 (w <= 56); a forward at
+ * 112 < h <= 128 runs, its backward is refused.  Shapes past the limits are refused before any launch.
  * fwd: out bf16 [B*N, heads*64], lse fp32 [B*heads, N] (log2 domain, nullable).
  * bwd: dqkv bf16 like qkv; dTh [2h-1,64], dTw [2w-1,64] fp32, added to (zero-initialise);
  *      scratch: delta [B*heads*N], relh_g [B*heads*Np*h], relw_g [B*heads*Np*w] (Np = N rounded up to 128), dt_ws
@@ -168,6 +170,9 @@ int pk_attn_bwd_saved(const void* qkv, const void* O, const void* dO, const floa
  * Decoder head (models_painter.py:328-333,430 decoder_pred = conv3x3 -> LayerNorm2D -> GELU -> conv1x1;
  * util/vitdet_utils.py:189-209) fused with forward_loss (:433-462) and patchify (:355-368).
  * g_nhwc: bf16 [B, H, W, 64] (output of the PK_EPI_PIXSHUF GEMM). wmat/wmat_t: pk_conv3x3_pack outputs.
+ * Image sizes: the conv runs on tiles of 128 pixels (wgrad: 64), min(W, 64) wide, which must tile the image: W a
+ * multiple of 64 with H even, or W < 64 dividing 64 with H a multiple of 128 / W.  Every decoder entry point
+ * refuses other sizes (W = 48 or 96, for example) before any launch.
  * head_params: fp32 [387] = conv3x3 bias[64] | LN2D weight[64] | LN2D bias[64] | conv1x1 weight[3][64] | bias[3].
  * fwd writes c1 (bf16 conv output, NHWC), patch_out fp32 [B, N, p*p*3] (= patchify(pred)), num[B] += sum
  * loss*mask*valid.  loss_kind: 0 smoothl1(beta .01), 1 l1, 2 l2, 3 l1l2.

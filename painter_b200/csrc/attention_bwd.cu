@@ -1278,6 +1278,9 @@ static int attn_bwd_impl(const void* qkv, const void* O, const void* dO, const f
   PK_CHECK(th_pad % 16 == 0 && tw_pad % 16 == 0 && th_pad >= 2 * h - 1 && tw_pad >= 2 * w - 1 &&
                th_pad <= 224 && tw_pad <= 112,
            "pk_attn_bwd: bad table padding th_pad=%d tw_pad=%d (h=%d w=%d)", th_pad, tw_pad, h, w);
+  // checked here, not only at the kernel switch below: the delta kernel is launched before it
+  PK_CHECK(w == 2 || w == 4 || w == 7 || w == 8 || w == 14 || w == 28 || w == 56,
+           "pk_attn_bwd: token-grid width %d unsupported (must divide 112)", w);
   const int N = h * w, C = heads * 64;
   AttnBwdArgs a;
   a.h = h; a.N = N; a.heads = heads; a.th_pad = th_pad; a.tw_pad = tw_pad;

@@ -503,6 +503,8 @@ extern "C" int pk_decoder_head_bwd(const void* c1, const float* tgts, const uint
            "pk_decoder_head_bwd: null pointer");
   PK_CHECK(W % 4 == 0 && static_cast<long long>(B) * H * W < (1ll << 31),
            "pk_decoder_head_bwd: W must be a multiple of 4 and B*H*W < 2^31");
+  int TW, TH;   // the image sizes the forward (pk_decoder_head_fwd) accepts
+  PK_CHECK(conv_tile_geometry(H, W, 128, &TW, &TH), "pk_decoder_head_bwd: unsupported image size %dx%d", H, W);
   if (g_head_bwd_legacy) {
     const int grid = sm_count() * 4;
     head_bwd_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(

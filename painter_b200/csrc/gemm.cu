@@ -283,16 +283,6 @@ static int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, GemmArgs&
   return 0;
 }
 
-static bool conv_tile_geometry(int H, int W, int pixels, int* TW, int* TH) {
-  int tw = W < 64 ? W : 64;
-  if (W % tw != 0 || pixels % tw != 0) return false;
-  int th = pixels / tw;
-  if (H % th != 0) return false;
-  *TW = tw;
-  *TH = th;
-  return true;
-}
-
 }  // namespace pk
 
 // test hooks: force the N tile (64/128/256) / the split-K factor; 0 restores the heuristics

@@ -63,6 +63,19 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   return cudaLaunchKernelEx(&L.cfg, kernel, std::forward<Args>(args)...);
 }
 
+// Tile of the decoder's implicit-GEMM 3x3 convolution: `pixels` pixels as TW = min(W, 64) columns x TH rows, which
+// must divide the W x H image (pixels = 128 for the forward / dgrad, 64 for the wgrad).  Every entry point that
+// handles the conv output checks it, so that all of them accept the same image sizes.
+inline bool conv_tile_geometry(int H, int W, int pixels, int* TW, int* TH) {
+  const int tw = W < 64 ? W : 64;
+  if (tw <= 0 || W % tw != 0 || pixels % tw != 0) return false;
+  const int th = pixels / tw;
+  if (H <= 0 || H % th != 0) return false;
+  *TW = tw;
+  *TH = th;
+  return true;
+}
+
 #define PK_CHECK(cond, ...)      \
   do {                           \
     if (!(cond)) {               \
